@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/sec of the TLS scan-to-map registration hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 2 -- a KITTI-seq00-shaped synthetic stream, 64-beam / 120k-pt
 scans reduced to F = 40 000 features (edge 8 000 / sphere 1 600 / planar 16 800 / ground 13 600) against an
@@ -38,6 +38,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the bench writes nothing into the tree it runs from (which may be read-only)
 
 METRIC = "frames/sec (120k-pt HDL-64 scan, 40k features) at 1/2/4/8 B200 vs CPU ref"
 UNIT = "frames/s"
@@ -90,6 +91,14 @@ def first_predict(fr):
 def pose_err(A, B):
     d = np.linalg.inv(A) @ B
     return float(np.linalg.norm(d[:3, 3])), float(np.arccos(np.clip((np.trace(d[:3, :3]) - 1) / 2, -1, 1)))
+
+
+def dump_outputs(dirname, **arrays):
+    """--dump-outputs: what the timed path returned to its caller in its last step, one DIR/<name>.npy (float64) per
+    array, so that two builds run with the same arguments (hence the same seeded inputs) can be compared."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 class ClockSampler:
@@ -472,6 +481,8 @@ def reference_arm(args, rank, world):
                 per_frame.append(dt)
                 stage += [st.t_kdtree, st.t_factors, st.t_solve, st.t_weights]
             last, cur = (cur if cur is not None else prev_gt), T
+        if mode == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, pose=T)
         med = float(np.median(per_frame))                    # per-frame MEDIAN: one descheduled frame does not move it
         results[mode] = (1.0 / med, 1e3 * med, (1e3 * stage / args.steps).tolist(), 1e3 * float(np.mean(per_frame)))
         if mode == 0 and args.steps * results[0][1] > 120e3:
@@ -553,6 +564,8 @@ def bench_config3(args, rank, world, local_rank):
     ms_e2e, T2, _ = run("host", args.warmup, args.steps)
     clocks = sampler.stop()
     assert np.array_equal(T, T2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pose=T)
     ms_dev = float(np.median(passes))
     reg.set_profiling(True)
     run("device", 0, 3)
@@ -611,6 +624,8 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=[2, 3],
                     help="BASELINE config: 2 = the headline stream (default); 3 = dense indoor scan, F=500k planar-only vs M=2M (N=1)")
     ap.add_argument("--batch", type=int, default=8, help="sequences per batched launch in the `batched` leg (0 = skip; N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the pose the last timed step returned (rank 0) as DIR/pose.npy, float64 4x4")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
 
@@ -685,6 +700,8 @@ def main():
         ms_dev, ms_e2e, ms_pageable = float(t[0]), float(t[1]), float(t[2])
     for a, b in zip(poses, poses_e2e):
         assert np.array_equal(a, b), "host-buffer and device-buffer paths disagree"
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, pose=poses[-1])
     gt_err = max(pose_err(T, fr["T_gt"])[0] for T, fr in zip(poses, frames))
 
     # ---- (f)-1: same stream with the map maintained on the device (informational; the headline stays `e2e`) ----

@@ -6,10 +6,12 @@ the strongest checks available in this image (VERDICT r1, "pin what can be pinne
     (dogleg_strategy.cc MakePolynomialForBoundaryConstrainedProblem / FindMinimumOnTrustRegionBoundary), via numpy.roots;
   * the converged pose of a fixed-correspondence, plane-only problem against scipy.optimize.least_squares(loss='cauchy')
     (same objective: 1/2 sum log(1 + r_i^2), 1-D residual blocks) and first-order optimality by finite differences;
-  * exact kNN against FLANN (cv2.flann, exhaustive checks) besides cKDTree;
+  * exact kNN against FLANN (cv2.flann, exhaustive checks; answers recorded in tests/golden/opencv_pins.npz) besides cKDTree;
   * the trust-region bookkeeping under a SMALL initial radius (dogleg boundary steps, rejected steps, radius updates):
     invariants that hold for Ceres' DoglegStrategy whatever the problem.
 """
+import os
+
 import numpy as np
 import pytest
 import scipy.optimize
@@ -113,13 +115,10 @@ def test_fixed_correspondence_solve_against_scipy_cauchy_least_squares(oracle):
 
 
 def test_knn_against_flann_exhaustive(oracle):
-    cv2 = pytest.importorskip("cv2")
-    rng = np.random.default_rng(5)
-    pts = rng.uniform(-20, 20, (4000, 3)).astype(np.float32)
-    qs = rng.uniform(-20, 20, (500, 3)).astype(np.float32)
-    # FLANN_INDEX_KDTREE_SINGLE (= flann::KDTreeSingleIndexParams, the exact tree Open3D's KDTreeFlann builds)
-    index = cv2.flann_Index(pts, dict(algorithm=4))
-    idx_f, d2_f = index.knnSearch(qs, 5, params=dict(checks=-1))
+    # FLANN_INDEX_KDTREE_SINGLE (= flann::KDTreeSingleIndexParams, the exact tree Open3D's KDTreeFlann builds), exhaustive
+    # checks, through OpenCV: its answers are recorded in tests/golden/opencv_pins.npz (tools/make_golden.py opencv)
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "opencv_pins.npz"))
+    pts, qs, idx_f, d2_f = g["knn_points"], g["knn_queries"], g["flann_idx"], g["flann_d2"]
     r = 3.0
     idx, d2, cnt = oracle.knn(pts.astype(np.float64), qs.astype(np.float64), r, 5)
     for i in range(len(qs)):

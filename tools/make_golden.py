@@ -4,7 +4,8 @@ The reference has no golden vectors of its own and cannot be run here (DESIGN.md
 pin the ORACLE (a regression guard for the checker) and give the GPU tests a fixture that does not depend on
 re-running the oracle.  Re-run this script only when the oracle is deliberately changed.
 
-    python tools/make_golden.py
+    python tools/make_golden.py            # tls_small.npz, feature_small.npz
+    python tools/make_golden.py opencv     # opencv_pins.npz (needs OpenCV's Python package)
 """
 import os
 import sys
@@ -89,5 +90,32 @@ def feature_golden():
     print(path, os.path.getsize(path), "bytes; lists:", [len(x) for x in lists])
 
 
+def opencv_golden():
+    """tests/golden/opencv_pins.npz: what OpenCV answers for the inputs of the two oracle pins that restate it --
+    cv2.fastAtan2 (groundRemove's angle) and exact FLANN kNN (FLANN_INDEX_KDTREE_SINGLE, the tree Open3D's
+    KDTreeFlann builds).  OpenCV is needed only to make this file, not to run the tests.
+
+        python tools/make_golden.py opencv
+    """
+    import cv2
+    rng = np.random.default_rng(0)
+    ys = np.concatenate([rng.normal(0, 20, 4000), [0.0, 0.0, 1.0, -1.0, 1e-30, -1e-30, 3.0, -3.0]]).astype(np.float32)
+    xs = np.concatenate([rng.normal(0, 20, 4000), [0.0, 1.0, 0.0, 0.0, 5.0, 5.0, 1e-30, -1e-30]]).astype(np.float32)
+    atan = np.array([cv2.fastAtan2(float(y), float(x)) for y, x in zip(ys, xs)], dtype=np.float32)
+    rng = np.random.default_rng(5)
+    pts = rng.uniform(-20, 20, (4000, 3)).astype(np.float32)
+    qs = rng.uniform(-20, 20, (500, 3)).astype(np.float32)
+    index = cv2.flann_Index(pts, dict(algorithm=4))
+    idx, d2 = index.knnSearch(qs, 5, params=dict(checks=-1))
+    out = {"atan_y": ys, "atan_x": xs, "fast_atan2": atan, "knn_points": pts, "knn_queries": qs,
+           "flann_idx": idx.astype(np.int32), "flann_d2": d2.astype(np.float32), "opencv_version": cv2.__version__}
+    path = os.path.join(ROOT, "tests", "golden", "opencv_pins.npz")
+    np.savez_compressed(path, **out)
+    print(path, os.path.getsize(path), "bytes; OpenCV", cv2.__version__)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["opencv"]:
+        opencv_golden()
+    else:
+        main()
